@@ -449,6 +449,30 @@ def secondary_metrics(dev, base_model, peak_tf, peak_hbm):
     return out
 
 
+DUMP_SAMPLE = 1 << 16  # elements kept per parameter tensor in --dump-outputs
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, model, losses):
+    """Writes what the timed train step leaves its caller after the last timed step, as float32 .npy files: the loss of
+    every step of the last timed loop (losses.npy) and every updated parameter (param.<name>.npy; tensors larger than
+    DUMP_SAMPLE elements as the same fixed, seeded sample of positions in every run).  About 15 MB for the base model."""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    arrays = {"losses": np.asarray(losses, dtype=np.float32)}
+    for name, p in model.named_parameters():
+        flat = p.detach().float().flatten()
+        if flat.numel() > DUMP_SAMPLE:
+            idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+            flat = flat[idx.to(flat.device)]
+        arrays[f"param.{name}"] = flat.cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT_BYTES, total
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -477,6 +501,9 @@ def main():
                     help="programmatic dependent launch for the library's kernels (default: the library's own default / MUSE_B200_PDL)")
     ap.add_argument("--ref-device", default="cpu", choices=["cpu", "cuda"],
                     help="--impl reference only: cpu (the reference arm) or cuda (same eager ops under bf16 autocast, informational)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the losses of the last timed loop and (a seeded sample of) the updated "
+                         "parameters as DIR/<name>.npy (float32), to compare two builds output for output")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -639,6 +666,8 @@ def main():
     ms_e2e = timed(e2e_step, args.steps)
     assert len(seen) == args.steps and all(math.isfinite(v) for v in seen), seen
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:  # before the profiled steps below move the parameters again
+        dump_outputs(args.dump_outputs, model, seen)
     model._packed.key = None  # graph replays update the parameters without bumping their version counters: re-pack for eager use
 
     # ---- roofline of the dominant kernel (tcgen05 GEMM), measured live with CUDA events around every launch

@@ -539,6 +539,159 @@ def make_uvit_schedules(muse):
     print("micro uvit v2 generate2 variants:", {k: v[0, :5].tolist() for k, v in out.items()})
 
 
+def make_sampling(muse):
+    """muse/sampling.py function by function on seeded inputs (tests/test_sampling_helpers_cpu.py): the public names, every
+    mask schedule of get_mask_chedule (or the exception it raises), mask_by_random_topk, top_k, log and the Gumbel helpers."""
+    import importlib
+
+    ref = importlib.import_module("muse.sampling")
+    names = sorted(n for n in dir(ref) if not n.startswith("_") and callable(getattr(ref, n)) and n not in ("partial",))
+    t = torch.linspace(0, 1, 21)
+    schedules = {}
+    for method in ("cosine", "linear", "sigmoid", "pow2", "pow3", "pow0.5", "pow", "log", "nonsense"):
+        try:
+            schedules[method] = ref.get_mask_chedule(method)(t)
+        except Exception as e:  # noqa: BLE001
+            schedules[method] = type(e).__name__
+    g = torch.Generator().manual_seed(0)
+    probs = torch.rand(3, 16, generator=g)
+    mask_len = torch.tensor([[3], [5], [1]])
+    x = torch.randn(2, 5, 16, generator=g)
+    t9 = torch.rand(9, generator=g)
+    out = dict(
+        mask_by_random_topk={temp: ref.mask_by_random_topk(mask_len, probs, temperature=temp,
+                                                           generator=torch.Generator().manual_seed(1))
+                             for temp in (0.0, 0.7, 4.0)},
+        top_k_07=ref.top_k(x, 0.7), top_k=ref.top_k(x), log=ref.log(probs),
+        gumbel_noise=ref.gumbel_noise(probs, generator=torch.Generator().manual_seed(2)),
+        gumbel_sample=ref.gumbel_sample(x, temperature=0.5, generator=torch.Generator().manual_seed(3)),
+        cosine_schedule=ref.cosine_schedule(t9), linear_schedule=ref.linear_schedule(t9),
+        sigmoid_schedule=ref.sigmoid_schedule(t9), pow=ref.pow(t9, "pow2.5"))
+    torch.save(dict(public_names=names, schedule_t=t, schedules=schedules, probs=probs, mask_len=mask_len, x=x, t=t9,
+                    outputs=out), os.path.join(HERE, "ref_sampling.pt"))
+    print("sampling:", len(names), "public names,", {k: v for k, v in schedules.items() if isinstance(v, str)})
+
+
+def make_lr_schedulers(muse):
+    """muse/lr_schedulers.py: 12 steps of every schedule name through get_scheduler (3 warm-up of 10 training steps) and of
+    the named constructors with non-default arguments, plus the SchedulerType values (tests/test_train_script_cpu.py)."""
+    import importlib
+    import json
+
+    sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
+    from tests.test_train_script_cpu import LR_CASES, _lr_sequence
+
+    ref = importlib.import_module("muse.lr_schedulers")
+    names = [e.value for e in ref.SchedulerType]
+    by_name = {n: _lr_sequence(lambda o: ref.get_scheduler(n, optimizer=o, num_warmup_steps=3, num_training_steps=10))
+               for n in names}
+    cases = [[fn, kw, _lr_sequence(lambda o: getattr(ref, fn)(o, **kw))] for fn, kw in LR_CASES]
+    with open(os.path.join(HERE, "ref_lr_schedulers.json"), "w") as f:
+        json.dump(dict(scheduler_types=names, get_scheduler=by_name, constructors=cases), f, indent=1)
+    print("lr schedulers:", names)
+
+
+def make_training_utils(muse):
+    """muse/training_utils.py: the logging diagnostics train_muse.py computes from the logits, on a seeded batch whose
+    masking rate spans every bucket (tests/test_train_muse_script_cpu.py)."""
+    import importlib
+
+    ref = importlib.import_module("muse.training_utils")
+    g = torch.Generator().manual_seed(0)
+    B, S, V = 12, 40, 16
+    logits = torch.randn(B, S, V, generator=g)
+    ids = torch.randint(0, V, (B, S), generator=g)
+    mask = torch.rand(B, S, generator=g) < torch.linspace(0.02, 1.0, B)[:, None]
+    mask[:, 0] = True
+    inp, lab = torch.where(mask, V, ids), torch.where(mask, ids, -100)
+    df = ref.token_probability_distributions_per_percent_masked_bucket(logits, inp, V)
+    torch.save(dict(mask_id=V, label_smoothing=0.1, logits=logits, input_ids=inp, labels=lab,
+                    buckets=ref.input_ids_to_masked_buckets(inp, V),
+                    pixel_entropy=ref.pixel_entropy_per_percent_masked_bucket(logits.clone(), inp.clone(), V),
+                    image_entropy=ref.image_entropy_per_percent_masked_bucket(logits.clone(), inp.clone(), V),
+                    cross_entropy=ref.cross_entropy_per_percent_masked_bucket(logits.clone(), lab.clone(), inp.clone(), V, V, 0.1),
+                    token_probs={"columns": list(df.columns), "dtypes": [str(d) for d in df.dtypes],
+                                 "values": {c: df[c].to_numpy() for c in df.columns}}),
+               os.path.join(HERE, "ref_training_utils.pt"))
+    print("training utils: token-probability rows", len(df))
+
+
+def make_interchange(muse):
+    """Checkpoints written by the reference's save_pretrained for the four model classes of
+    tests/test_checkpoint_interchange_cpu.py: its config.json verbatim, the state-dict keys / shapes / dtypes in the order
+    torch.save wrote them, a SHA-256 of every tensor's bytes (the weights themselves are the seeded initialisation plus a
+    seeded perturbation, which the test redraws and checks against the digests) and the reference's forward output on the
+    test's seeded inputs."""
+    import json
+    import tempfile
+
+    from muse.modeling_transformer_v2 import MaskGiTUViT_v2
+
+    sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
+    from tests.test_checkpoint_interchange_cpu import KINDS, _digest, _inputs
+
+    classes = {"MaskGitTransformer": muse.MaskGitTransformer, "MaskGiTUViT_v2": MaskGiTUViT_v2,
+               "MaskGitVQGAN": muse.MaskGitVQGAN, "VQGANModel": muse.VQGANModel}
+    out = {}
+    for kind, cfg in KINDS:
+        torch.manual_seed(1234)
+        r = classes[kind](**cfg)
+        with torch.no_grad():
+            for p in r.parameters():
+                p.add_((0.1 if p.dim() == 1 else 0.02) * torch.randn_like(p))
+        r.eval()
+        inputs = _inputs(kind)
+        with tempfile.TemporaryDirectory() as d:
+            r.save_pretrained(d)
+            config_json = open(os.path.join(d, "config.json")).read()
+            saved = torch.load(os.path.join(d, "pytorch_model.bin"))
+        with torch.no_grad():
+            if kind == "MaskGitTransformer":
+                y = r(inputs["input_ids"])
+            elif kind == "MaskGiTUViT_v2":
+                y = r(inputs["input_ids"], inputs["enc"], inputs["cond"], inputs["micro"])
+            else:
+                y = r.decode_code(r.get_code(inputs["image"]))
+        out[kind] = dict(config=cfg, config_json=json.loads(config_json),
+                         keys=[(k, list(v.shape), str(v.dtype), _digest(v)) for k, v in saved.items()],
+                         output=y.clone())
+    torch.save(out, os.path.join(HERE, "ref_interchange.pt"))
+    print("interchange:", {k: len(v["keys"]) for k, v in out.items()})
+
+
+def make_surface(muse):
+    """The public surface of the reference classes (tests/test_checkpoint_interchange_cpu.py): public class attributes beyond
+    torch.nn.Module's, public instance attributes, config keys in order and the module tree (names, order)."""
+    import json
+
+    from muse.modeling_transformer_v2 import MaskGiTUViT_v2
+
+    base = set(dir(torch.nn.Module))
+    v1 = dict(vocab_size=72, hidden_size=64, num_hidden_layers=1, num_attention_heads=1, intermediate_size=128,
+              add_cross_attention=True, encoder_hidden_size=32, project_encoder_hidden_states=True)
+    v2 = dict(hidden_size=128, num_attention_heads=2, in_channels=64, block_out_channels=(64,), block_num_heads=1,
+              num_res_blocks=1, num_hidden_layers=1, intermediate_size=128, vocab_size=72, codebook_size=64,
+              encoder_hidden_size=32, cond_embed_dim=16, micro_cond_encode_dim=8, micro_cond_embed_dim=40)
+    vq = dict(resolution=32, hidden_channels=32, channel_mult=(1, 2), num_res_blocks=1, z_channels=16, num_embeddings=64,
+              quantized_embed_dim=16)
+    table = {}
+    for name, cls, kw in (("MaskGitTransformer", muse.MaskGitTransformer, v1), ("MaskGiTUViT_v2", MaskGiTUViT_v2, v2),
+                          ("MaskGitVQGAN", muse.MaskGitVQGAN, vq), ("VQGANModel", muse.VQGANModel, vq),
+                          ("EMAModel", muse.EMAModel, None), ("PipelineMuse", muse.PipelineMuse, None),
+                          ("PipelineMuseInpainting", muse.PipelineMuseInpainting, None)):
+        row = {"class_attributes": sorted({a for a in dir(cls) if not a.startswith("_")} - base), "kwargs": kw}
+        if kw is not None:
+            with torch.device("meta"):
+                m = cls(**kw)
+            row["instance_attributes"] = sorted(k for k in vars(m) if not k.startswith("_"))
+            row["config_keys"] = list(m.config.keys())
+            row["module_tree"] = [n for n, _ in m.named_modules()]
+        table[name] = row
+    with open(os.path.join(HERE, "ref_surface.json"), "w") as f:
+        json.dump(table, f, indent=1)
+    print("surface:", {k: len(v["class_attributes"]) for k, v in table.items()})
+
+
 def main():
     muse = import_reference()
     torch.set_num_threads(4)
@@ -569,6 +722,16 @@ def main():
             make_uvit_grads(muse)
         if "uvit_schedules" in only[0]:
             make_uvit_schedules(muse)
+        if "sampling" in only[0]:
+            make_sampling(muse)
+        if "lr_schedulers" in only[0]:
+            make_lr_schedulers(muse)
+        if "training_utils" in only[0]:
+            make_training_utils(muse)
+        if "interchange" in only[0]:
+            make_interchange(muse)
+        if "surface" in only[0]:
+            make_surface(muse)
         return
 
     # ---- (1) micro class-conditional transformer: weights + inputs + logits/loss/all grads
@@ -793,6 +956,11 @@ def main():
     make_uvit_schedules(muse)
     make_pipeline_text(muse)
     make_inpainting_text(muse)
+    make_sampling(muse)
+    make_lr_schedulers(muse)
+    make_training_utils(muse)
+    make_interchange(muse)
+    make_surface(muse)
 
     for f in sorted(os.listdir(HERE)):
         if f.endswith(".pt"):

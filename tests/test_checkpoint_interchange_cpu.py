@@ -1,21 +1,21 @@
-"""Checkpoints cross the boundary in BOTH directions (no GPU): a model saved by this package's ``save_pretrained`` loads into
-the UNMODIFIED reference class with ``from_pretrained`` (every key consumed, none missing), and a model saved by the reference
-loads here -- ``config.json`` keys, ``pytorch_model.bin`` names and shapes are the compatibility contract (SURVEY 8b).  The
-reference runs in a subprocess (its package is also called ``muse``); the forward of the loaded weights is then compared
+"""Checkpoints cross the boundary in BOTH directions (no GPU): a model saved by this package's ``save_pretrained`` writes the
+config.json and the state-dict keys, shapes and dtypes the UNMODIFIED reference class writes for the same configuration (so
+its ``from_pretrained`` consumes every key), and a model saved by the reference loads here -- ``config.json`` keys,
+``pytorch_model.bin`` names and shapes are the compatibility contract (SURVEY 8b).  What the reference wrote is stored in
+tests/golden/ref_interchange.pt (make_golden.py::make_interchange): its config.json, its state-dict layout with a SHA-256 of
+every tensor, and its forward output.  Its weights are the seeded initialisation plus a seeded perturbation; they are redrawn
+here, checked against the digests and written in the reference's key order.  The forward of the loaded weights is compared
 numerically: the reference's own CPU forward against this package's host code on the kernels' torch restatements."""
+import hashlib
 import json
 import os
-import subprocess
-import sys
 
 import pytest
 import torch
 
-from oracle import ref_snapshot
 from tests import cpu_math_ops
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-pytestmark = pytest.mark.skipif(not ref_snapshot.available(), reason="oracle/_ref snapshot of the reference not available")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 V1 = dict(vocab_size=72, hidden_size=64, num_hidden_layers=2, num_attention_heads=1, intermediate_size=128, hidden_dropout=0.0,
           attention_dropout=0.0, max_position_embeddings=17, codebook_size=64, num_vq_tokens=16, num_classes=7)
@@ -26,42 +26,9 @@ VQ = dict(resolution=32, num_channels=3, hidden_channels=32, channel_mult=[1, 2]
           num_embeddings=64, quantized_embed_dim=16)
 TVQ = dict(VQ, num_res_blocks=2, attn_resolutions=[16])
 
-REF_SIDE = r'''
-import json, sys, torch
-sys.path.insert(0, sys.argv[1])
-from oracle.ref_snapshot import import_reference
-muse = import_reference()
-from muse.modeling_transformer_v2 import MaskGiTUViT_v2
-classes = {"MaskGitTransformer": muse.MaskGitTransformer, "MaskGiTUViT_v2": MaskGiTUViT_v2, "MaskGitVQGAN": muse.MaskGitVQGAN,
-           "VQGANModel": muse.VQGANModel}
-for kind, base in json.load(open(sys.argv[2])):  # one job per model class: <base>/{ours, theirs, inputs.pt, cfg.json}
-    cls = classes[kind]
-    dir_a, dir_b = base + "/ours", base + "/theirs"
-    inputs = torch.load(base + "/inputs.pt")
-    # (1) what this package saved loads into the unmodified reference class
-    m = cls.from_pretrained(dir_a, low_cpu_mem_usage=False)
-    saved = torch.load(dir_a + "/pytorch_model.bin")
-    sd = m.state_dict()
-    assert list(sd) == list(saved), (kind, set(sd) ^ set(saved))
-    assert all(torch.equal(sd[k], saved[k]) for k in sd), kind
-    # (2) a differently seeded reference model, saved by the reference, with its own forward output
-    torch.manual_seed(1234)
-    r = cls(**json.load(open(base + "/cfg.json")))
-    with torch.no_grad():
-        for p in r.parameters():  # every tensor non-trivial (norm weights are ones, adaLN mappers and GRN parameters zeros at init)
-            p.add_((0.1 if p.dim() == 1 else 0.02) * torch.randn_like(p))
-    r.eval()
-    r.save_pretrained(dir_b)
-    with torch.no_grad():
-        if kind == "MaskGitTransformer":
-            out = r(inputs["input_ids"])
-        elif kind == "MaskGiTUViT_v2":
-            out = r(inputs["input_ids"], inputs["enc"], inputs["cond"], inputs["micro"])
-        else:
-            out = r.decode_code(r.get_code(inputs["image"]))
-    torch.save(out, dir_b + "/reference_output.pt")
-print("OK")
-'''
+
+def _digest(t):
+    return hashlib.sha256(t.detach().contiguous().cpu().numpy().tobytes()).hexdigest()
 
 
 def _inputs(kind):
@@ -79,26 +46,39 @@ KINDS = [("MaskGitTransformer", V1), ("MaskGiTUViT_v2", V2), ("MaskGitVQGAN", VQ
 
 @pytest.fixture(scope="module")
 def exchanged(tmp_path_factory):
-    """this package saves one model per class, ONE reference subprocess loads them all and saves its own"""
+    """this package saves one model per class and checks it against the reference's layout; the reference's checkpoint of
+    each class is re-materialised from the golden file"""
     import open_muse_b200 as ours
 
+    ref = torch.load(os.path.join(GOLDEN, "ref_interchange.pt"), weights_only=False)
     root = tmp_path_factory.mktemp("interchange")
-    jobs = []
+    dirs = {}
     for kind, cfg in KINDS:
+        r = ref[kind]
+        assert r["config"] == cfg, kind
         base = str(root / kind)
-        os.makedirs(base)
+        # (1) what this package saves is what the unmodified reference class saves and loads: config and state-dict layout
         torch.manual_seed(99)
         getattr(ours, kind)(**cfg).save_pretrained(os.path.join(base, "ours"))
-        torch.save(_inputs(kind), os.path.join(base, "inputs.pt"))
-        with open(os.path.join(base, "cfg.json"), "w") as f:
-            json.dump(cfg, f)
-        jobs.append((kind, base))
-    with open(root / "jobs.json", "w") as f:
-        json.dump(jobs, f)
-    r = subprocess.run([sys.executable, "-c", REF_SIDE, ROOT, str(root / "jobs.json")], capture_output=True, text=True,
-                       timeout=900, env=dict(os.environ, OMP_NUM_THREADS="4"))
-    assert r.returncode == 0 and r.stdout.strip().endswith("OK"), r.stderr[-3000:]
-    return dict(jobs)
+        assert json.load(open(os.path.join(base, "ours", "config.json"))) == r["config_json"], kind
+        saved = torch.load(os.path.join(base, "ours", "pytorch_model.bin"))
+        assert [(k, list(v.shape), str(v.dtype)) for k, v in saved.items()] == [tuple(x[:3]) for x in r["keys"]], kind
+        # (2) the reference's checkpoint: its weights redrawn bit for bit, its key order, its config.json
+        torch.manual_seed(1234)
+        m = getattr(ours, kind)(**cfg)
+        with torch.no_grad():
+            for p in m.parameters():  # every tensor non-trivial (norm weights are ones, adaLN mappers and GRN parameters zeros at init)
+                p.add_((0.1 if p.dim() == 1 else 0.02) * torch.randn_like(p))
+        sd = m.state_dict()
+        assert [k for k, v in sd.items() if _digest(v) != dict((x[0], x[3]) for x in r["keys"]).get(k)] == [], kind
+        dir_b = os.path.join(base, "theirs")
+        os.makedirs(dir_b)
+        torch.save({k: sd[k] for k, *_ in r["keys"]}, os.path.join(dir_b, "pytorch_model.bin"))
+        with open(os.path.join(dir_b, "config.json"), "w") as f:
+            json.dump(r["config_json"], f)
+        torch.save(r["output"], os.path.join(dir_b, "reference_output.pt"))
+        dirs[kind] = base
+    return dirs
 
 
 @pytest.mark.parametrize("kind,cfg", KINDS)
@@ -132,46 +112,30 @@ def test_checkpoints_are_interchangeable_with_the_unmodified_reference(exchanged
     assert float((got.float() - want).norm() / want.norm()) < (5e-5 if "VQ" not in kind else 1e-3)
 
 
-SURFACE_SIDE = r'''
-import sys, torch
-sys.path.insert(0, sys.argv[1])
-from oracle.ref_snapshot import import_reference
-ref = import_reference()
-from muse.modeling_transformer_v2 import MaskGiTUViT_v2 as RefV2
-import open_muse_b200 as ours
-base = set(dir(torch.nn.Module))
-V1 = dict(vocab_size=72, hidden_size=64, num_hidden_layers=1, num_attention_heads=1, intermediate_size=128, add_cross_attention=True,
-          encoder_hidden_size=32, project_encoder_hidden_states=True)
-V2 = dict(hidden_size=128, num_attention_heads=2, in_channels=64, block_out_channels=(64,), block_num_heads=1, num_res_blocks=1,
-          num_hidden_layers=1, intermediate_size=128, vocab_size=72, codebook_size=64, encoder_hidden_size=32, cond_embed_dim=16,
-          micro_cond_encode_dim=8, micro_cond_embed_dim=40)
-VQ = dict(resolution=32, hidden_channels=32, channel_mult=(1, 2), num_res_blocks=1, z_channels=16, num_embeddings=64,
-          quantized_embed_dim=16)
-bad = []
-for name, r, o, kw in (("MaskGitTransformer", ref.MaskGitTransformer, ours.MaskGitTransformer, V1), ("MaskGiTUViT_v2", RefV2, ours.MaskGiTUViT_v2, V2),
-                       ("MaskGitVQGAN", ref.MaskGitVQGAN, ours.MaskGitVQGAN, VQ), ("VQGANModel", ref.VQGANModel, ours.VQGANModel, VQ),
-                       ("EMAModel", ref.EMAModel, ours.EMAModel, None), ("PipelineMuse", ref.PipelineMuse, ours.PipelineMuse, None),
-                       ("PipelineMuseInpainting", ref.PipelineMuseInpainting, ours.PipelineMuseInpainting, None)):
-    missing = ({a for a in dir(r) if not a.startswith("_")} - base) - {a for a in dir(o) if not a.startswith("_")}
-    if missing:
-        bad.append((name, "class attributes", sorted(missing)))
-    if kw is None:
-        continue
-    with torch.device("meta"):
-        a, b = r(**kw), o(**kw)
-    missing = {k for k in vars(a) if not k.startswith("_")} - {k for k in vars(b) if not k.startswith("_")}
-    if missing:
-        bad.append((name, "instance attributes", sorted(missing)))
-    if list(a.config.keys()) != list(b.config.keys()):
-        bad.append((name, "config keys", sorted(set(a.config.keys()) ^ set(b.config.keys()))))
-    if [n for n, _ in a.named_modules()] != [n for n, _ in b.named_modules()]:
-        bad.append((name, "module tree", "differs"))
-print("BAD", bad) if bad else print("OK")
-'''
-
-
 def test_public_surface_of_every_class_covers_the_reference():
     """every public class attribute / method, every public instance attribute, the config keys in order and the module tree
-    (names, order) of the reference classes exist on the drop-in classes (reference imported in a subprocess)"""
-    r = subprocess.run([sys.executable, "-c", SURFACE_SIDE, ROOT], capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0 and r.stdout.strip().endswith("OK"), (r.stdout[-2000:], r.stderr[-2000:])
+    (names, order) of the reference classes exist on the drop-in classes (the reference's surface is stored in
+    tests/golden/ref_surface.json by make_golden.py::make_surface)"""
+    import open_muse_b200 as ours
+
+    with open(os.path.join(GOLDEN, "ref_surface.json")) as f:
+        ref = json.load(f)
+    base = set(dir(torch.nn.Module))
+    bad = []
+    for name, r in ref.items():
+        o = getattr(ours, name)
+        missing = set(r["class_attributes"]) - base - {a for a in dir(o) if not a.startswith("_")}
+        if missing:
+            bad.append((name, "class attributes", sorted(missing)))
+        if r["kwargs"] is None:
+            continue
+        with torch.device("meta"):
+            b = o(**r["kwargs"])
+        missing = set(r["instance_attributes"]) - {k for k in vars(b) if not k.startswith("_")}
+        if missing:
+            bad.append((name, "instance attributes", sorted(missing)))
+        if r["config_keys"] != list(b.config.keys()):
+            bad.append((name, "config keys", sorted(set(r["config_keys"]) ^ set(b.config.keys()))))
+        if r["module_tree"] != [n for n, _ in b.named_modules()]:
+            bad.append((name, "module tree", "differs"))
+    assert not bad, bad

@@ -1,62 +1,43 @@
 """``open_muse_b200.sampling`` (= ``muse.sampling`` of the drop-in package) against the reference module, function by function
 on seeded inputs: the mask schedules of ``get_mask_chedule`` (the training masking rate and generate2's re-mask schedule),
-``mask_by_random_topk`` through the same generator, ``top_k``, the Gumbel helpers.  The reference file is loaded by path (it
-has no package-relative imports); skipped where neither /root/reference nor the oracle/_ref snapshot exists."""
-import importlib.util
-import os
+``mask_by_random_topk`` through the same generator, ``top_k``, the Gumbel helpers.  What the reference returned (or raised)
+is stored in tests/golden/ref_sampling.pt (make_golden.py::make_sampling)."""
+import builtins
 
 import pytest
 import torch
 
 import open_muse_b200.sampling as mine
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-PATHS = [os.path.join(os.environ.get("MUSE_REFERENCE", "/root/reference"), "muse", "sampling.py"),
-         os.path.join(ROOT, "oracle", "_ref", "muse", "sampling.py")]
-PATH = next((p for p in PATHS if os.path.exists(p)), None)
-pytestmark = pytest.mark.skipif(PATH is None, reason="reference muse/sampling.py not available")
-
 
 @pytest.fixture(scope="module")
-def ref():
-    spec = importlib.util.spec_from_file_location("_ref_sampling", PATH)
-    m = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(m)
-    return m
+def ref(golden):
+    return golden("ref_sampling.pt")
 
 
 def test_public_names(ref):
-    names = [n for n in dir(ref) if not n.startswith("_") and callable(getattr(ref, n)) and n not in ("partial",)]
-    assert all(hasattr(mine, n) for n in names), [n for n in names if not hasattr(mine, n)]
+    names = ref["public_names"]
+    assert names and all(hasattr(mine, n) for n in names), [n for n in names if not hasattr(mine, n)]
 
 
 @pytest.mark.parametrize("method", ["cosine", "linear", "sigmoid", "pow2", "pow3", "pow0.5", "pow", "log", "nonsense"])
 def test_mask_schedules(ref, method):
-    t = torch.linspace(0, 1, 21)
-    try:
-        want = ref.get_mask_chedule(method)(t)
-    except Exception as e:  # noqa: BLE001
-        with pytest.raises(type(e)):
+    t, want = ref["schedule_t"], ref["schedules"][method]
+    if isinstance(want, str):  # the reference raised this exception type
+        with pytest.raises(getattr(builtins, want)):
             mine.get_mask_chedule(method)(t)
         return
     torch.testing.assert_close(mine.get_mask_chedule(method)(t), want, rtol=0, atol=0, equal_nan=True)
 
 
 def test_sampling_helpers(ref):
-    g = torch.Generator().manual_seed(0)
-    probs = torch.rand(3, 16, generator=g)
-    mask_len = torch.tensor([[3], [5], [1]])
-    for temp in (0.0, 0.7, 4.0):
-        a = ref.mask_by_random_topk(mask_len, probs, temperature=temp, generator=torch.Generator().manual_seed(1))
-        b = mine.mask_by_random_topk(mask_len, probs, temperature=temp, generator=torch.Generator().manual_seed(1))
+    probs, x, t, want = ref["probs"], ref["x"], ref["t"], ref["outputs"]
+    for temp, a in want["mask_by_random_topk"].items():
+        b = mine.mask_by_random_topk(ref["mask_len"], probs, temperature=temp, generator=torch.Generator().manual_seed(1))
         assert torch.equal(a, b), temp
-    x = torch.randn(2, 5, 16, generator=g)
-    assert torch.equal(ref.top_k(x, 0.7), mine.top_k(x, 0.7)) and torch.equal(ref.top_k(x), mine.top_k(x))
-    assert torch.equal(ref.log(probs), mine.log(probs))
-    assert torch.equal(ref.gumbel_noise(probs, generator=torch.Generator().manual_seed(2)),
-                       mine.gumbel_noise(probs, generator=torch.Generator().manual_seed(2)))
-    assert torch.equal(ref.gumbel_sample(x, temperature=0.5, generator=torch.Generator().manual_seed(3)),
-                       mine.gumbel_sample(x, temperature=0.5, generator=torch.Generator().manual_seed(3)))
-    t = torch.rand(9, generator=g)
+    assert torch.equal(want["top_k_07"], mine.top_k(x, 0.7)) and torch.equal(want["top_k"], mine.top_k(x))
+    assert torch.equal(want["log"], mine.log(probs))
+    assert torch.equal(want["gumbel_noise"], mine.gumbel_noise(probs, generator=torch.Generator().manual_seed(2)))
+    assert torch.equal(want["gumbel_sample"], mine.gumbel_sample(x, temperature=0.5, generator=torch.Generator().manual_seed(3)))
     for fn, args in (("cosine_schedule", (t,)), ("linear_schedule", (t,)), ("sigmoid_schedule", (t,)), ("pow", (t, "pow2.5"))):
-        torch.testing.assert_close(getattr(mine, fn)(*args), getattr(ref, fn)(*args), rtol=0, atol=0)
+        torch.testing.assert_close(getattr(mine, fn)(*args), want[fn], rtol=0, atol=0)

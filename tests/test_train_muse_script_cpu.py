@@ -16,9 +16,10 @@ from tests import cpu_math_ops
 from tests.train_script_harness import find_script, make_muse_config, run_script
 
 SCRIPT = find_script("train_muse.py")
-pytestmark = pytest.mark.skipif(SCRIPT is None, reason="reference training script not available")
+needs_script = pytest.mark.skipif(SCRIPT is None, reason="reference training script not available")
 
 
+@needs_script
 @pytest.mark.parametrize("use_ema", [False, True])
 def test_reference_train_muse_script_runs_unchanged(monkeypatch, tmp_path, use_ema):
     cpu_math_ops.install(monkeypatch, exact=False)
@@ -52,16 +53,14 @@ def test_reference_train_muse_script_runs_unchanged(monkeypatch, tmp_path, use_e
 def test_training_utils_diagnostics_match_reference():
     """compat muse.training_utils (the logging diagnostics train_muse.py computes from the returned logits) against the
     reference's module, value for value -- including the upstream behaviour of scattering per-token cross-entropies with a
-    per-image index"""
-    import importlib.util
+    per-image index (the reference's values are stored in tests/golden/ref_training_utils.pt by
+    make_golden.py::make_training_utils)"""
     import sys
 
-    ref_path = os.path.join(os.path.dirname(os.path.dirname(SCRIPT)), "muse", "training_utils.py")
-    if not os.path.exists(ref_path):
-        pytest.skip("reference muse/ not available")
-    spec = importlib.util.spec_from_file_location("_ref_training_utils", ref_path)
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
+    import numpy as np
+
+    ref = torch.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_training_utils.pt"),
+                     weights_only=False)
     sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "open_muse_b200", "compat"))
     try:
         for k in [k for k in sys.modules if k == "muse" or k.startswith("muse.")]:
@@ -69,27 +68,24 @@ def test_training_utils_diagnostics_match_reference():
         from muse import training_utils as mine
     finally:
         sys.path.pop(0)
-    g = torch.Generator().manual_seed(0)
-    B, S, V = 12, 40, 16
-    logits = torch.randn(B, S, V, generator=g)
-    ids = torch.randint(0, V, (B, S), generator=g)
-    mask = torch.rand(B, S, generator=g) < torch.linspace(0.02, 1.0, B)[:, None]
-    mask[:, 0] = True
-    inp, lab = torch.where(mask, V, ids), torch.where(mask, ids, -100)
-    assert torch.equal(ref.input_ids_to_masked_buckets(inp, V), mine.input_ids_to_masked_buckets(inp, V))
-    for name, args in (("pixel_entropy_per_percent_masked_bucket", (logits, inp, V)),
-                       ("image_entropy_per_percent_masked_bucket", (logits, inp, V)),
-                       ("cross_entropy_per_percent_masked_bucket", (logits, lab, inp, V, V, 0.1))):
-        r = getattr(ref, name)(*[a.clone() if torch.is_tensor(a) else a for a in args])
+    logits, inp, lab, V = ref["logits"], ref["input_ids"], ref["labels"], ref["mask_id"]
+    assert torch.equal(ref["buckets"], mine.input_ids_to_masked_buckets(inp, V))
+    for key, name, args in (("pixel_entropy", "pixel_entropy_per_percent_masked_bucket", (logits, inp, V)),
+                            ("image_entropy", "image_entropy_per_percent_masked_bucket", (logits, inp, V)),
+                            ("cross_entropy", "cross_entropy_per_percent_masked_bucket",
+                             (logits, lab, inp, V, V, ref["label_smoothing"]))):
         m = getattr(mine, name)(*[a.clone() if torch.is_tensor(a) else a for a in args])
-        torch.testing.assert_close(m, r, rtol=1e-5, atol=1e-6)
-    r = ref.token_probability_distributions_per_percent_masked_bucket(logits, inp, V)
+        torch.testing.assert_close(m, ref[key], rtol=1e-5, atol=1e-6)
+    r = ref["token_probs"]
     m = mine.token_probability_distributions_per_percent_masked_bucket(logits, inp, V)
-    assert r.equals(m) and len(r) > 0
+    assert list(m.columns) == r["columns"] and [str(d) for d in m.dtypes] == r["dtypes"] and len(m) > 0
+    for c in r["columns"]:
+        assert np.array_equal(m[c].to_numpy(), r["values"][c]), c
     for k in [k for k in sys.modules if k == "muse" or k.startswith("muse.")]:
         del sys.modules[k]
 
 
+@needs_script
 def test_reference_train_muse_script_generates_and_inpaints_during_training(monkeypatch, tmp_path):
     """``experiment.generate_every`` of the unmodified train_muse.py: ``generate_images`` (16 validation prompts through the
     text encoder, classifier-free guidance against the encoded empty prompt, per-sample micro conditions, generate2 -> clamp ->
@@ -132,6 +128,7 @@ def test_reference_train_muse_script_generates_and_inpaints_during_training(monk
     assert sorted(inp[0]["captions"]) == ["a red cube", "two dogs"] and all(s == [64, 64] for s in inp[0]["sizes"])
 
 
+@needs_script
 def test_train_muse_script_cannot_train_the_v1_text_conditional_transformer_upstream(monkeypatch, tmp_path):
     """``architecture: transformer`` in train_muse.py = the text-conditional MaskGitTransformer (the model class of BASELINE
     config 4).  At this commit the UNMODIFIED script stops in its own code on both target modes, before or right after the
@@ -151,6 +148,7 @@ def test_train_muse_script_cannot_train_the_v1_text_conditional_transformer_upst
         run_script(SCRIPT, cfg, extra_cli=("training.use_soft_code_target=False",))
 
 
+@needs_script
 def test_reference_train_muse_script_resumes_with_ema(monkeypatch, tmp_path):
     """resume of the unmodified train_muse.py with EMA: ``accelerator.load_state`` runs the script's load hook
     (``EMAModel.from_pretrained(checkpoint/ema_model, model_cls=...)`` -> ``ema.load_state_dict`` -> ``ema.to``), the model /

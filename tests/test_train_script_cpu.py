@@ -14,7 +14,7 @@ from tests.train_script_harness import find_script, make_config, run_script
 from tests.test_v1_plumbing_cpu import _fake_ops
 
 SCRIPT = find_script()
-pytestmark = pytest.mark.skipif(SCRIPT is None, reason="reference training script not available")
+needs_script = pytest.mark.skipif(SCRIPT is None, reason="reference training script not available")
 
 
 def _fake_tokenizer(mp):
@@ -33,6 +33,7 @@ def _fake_tokenizer(mp):
     mp.setattr(V.MaskGitVQGAN, "get_soft_code", soft)
 
 
+@needs_script
 @pytest.mark.parametrize("soft_targets", [False, True])
 def test_reference_training_script_runs_unchanged(monkeypatch, tmp_path, soft_targets):
     _fake_ops(monkeypatch)
@@ -64,6 +65,7 @@ IMAGENET_YAML_TRANSFORMER = dict(
     use_mlm_layernorm=True, use_bias=False, hidden_dropout=0.0, attention_dropout=0.0)
 
 
+@needs_script
 def test_reference_training_script_with_its_own_imagenet_yaml_model(monkeypatch, tmp_path):
     """The same unmodified script with the transformer section of the reference's configs/imagenet.yaml (depth cut from 24 to 2
     layers for time): the constructor accepts head_dim 48 and the step loop runs (stand-in kernels; the kernels themselves are
@@ -87,66 +89,53 @@ def test_reference_training_script_with_its_own_imagenet_yaml_model(monkeypatch,
     assert cfg_json["hidden_size"] == 768 and cfg_json["num_attention_heads"] == 16 and cfg_json["mask_token_id"] == 2047
 
 
+def _lr_sequence(make):
+    opt = torch.optim.SGD([torch.nn.Parameter(torch.zeros(1))], lr=0.5)
+    sch = make(opt)
+    seq = []
+    for _ in range(12):
+        opt.step()
+        sch.step()
+        seq.append(sch.get_last_lr()[0])
+    return seq
+
+
+# the named constructors of the reference module with non-default arguments
+LR_CASES = [("get_cosine_schedule_with_warmup", dict(num_warmup_steps=2, num_training_steps=10, num_cycles=1.5)),
+            ("get_cosine_schedule_with_warmup", dict(num_warmup_steps=2, num_training_steps=10, num_cycles=1)),
+            ("get_cosine_with_hard_restarts_schedule_with_warmup", dict(num_warmup_steps=2, num_training_steps=10, num_cycles=3)),
+            ("get_polynomial_decay_schedule_with_warmup", dict(num_warmup_steps=2, num_training_steps=10, lr_end=1e-3, power=2.0)),
+            ("get_linear_schedule_with_warmup", dict(num_warmup_steps=2, num_training_steps=10)),
+            ("get_constant_schedule_with_warmup", dict(num_warmup_steps=2)), ("get_constant_schedule", {})]
+
+
 def test_lr_schedulers_match_reference():
-    """compat muse.lr_schedulers.get_scheduler against the reference's, every schedule name, 12 steps."""
-    import importlib.util
+    """compat muse.lr_schedulers.get_scheduler against the reference's, every schedule name, 12 steps (the reference's
+    learning rates are stored in tests/golden/ref_lr_schedulers.json by make_golden.py::make_lr_schedulers)."""
     import sys
 
-    ref_dir = os.path.join(os.path.dirname(os.path.dirname(SCRIPT)), "muse")
-    if not os.path.exists(os.path.join(ref_dir, "lr_schedulers.py")):
-        pytest.skip("reference muse/ not available")
-    import types
-
-    pkg = types.ModuleType("_ref_muse")
-    pkg.__path__ = [ref_dir]
-    sys.modules["_ref_muse"] = pkg
-    try:
-        spec = importlib.util.spec_from_file_location("_ref_muse.logging", os.path.join(ref_dir, "logging.py"))
-        lg = importlib.util.module_from_spec(spec); sys.modules["_ref_muse.logging"] = lg; spec.loader.exec_module(lg)
-        spec = importlib.util.spec_from_file_location("_ref_muse.lr_schedulers", os.path.join(ref_dir, "lr_schedulers.py"))
-        ref = importlib.util.module_from_spec(spec); sys.modules["_ref_muse.lr_schedulers"] = ref; spec.loader.exec_module(ref)
-    finally:
-        pass
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_lr_schedulers.json")) as f:
+        ref = json.load(f)
     sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "open_muse_b200", "compat"))
     try:
-        from muse.lr_schedulers import NAMES, get_scheduler
+        for k in [k for k in sys.modules if k == "muse" or k.startswith("muse.")]:
+            del sys.modules[k]
+        import muse.lr_schedulers as mine
     finally:
         sys.path.pop(0)
-    for name in NAMES:
-        lrs = []
-        for impl in (ref.get_scheduler, get_scheduler):
-            opt = torch.optim.SGD([torch.nn.Parameter(torch.zeros(1))], lr=0.5)
-            sch = impl(name, optimizer=opt, num_warmup_steps=3, num_training_steps=10)
-            seq = []
-            for _ in range(12):
-                opt.step(); sch.step(); seq.append(sch.get_last_lr()[0])
-            lrs.append(seq)
-        assert lrs[0] == pytest.approx(lrs[1], rel=1e-12, abs=1e-15), name
-    import muse.lr_schedulers as mine
-
-    # the named constructors and the enum of the reference module, with non-default arguments
-    cases = [("get_cosine_schedule_with_warmup", dict(num_warmup_steps=2, num_training_steps=10, num_cycles=1.5)),
-             ("get_cosine_schedule_with_warmup", dict(num_warmup_steps=2, num_training_steps=10, num_cycles=1)),
-             ("get_cosine_with_hard_restarts_schedule_with_warmup", dict(num_warmup_steps=2, num_training_steps=10, num_cycles=3)),
-             ("get_polynomial_decay_schedule_with_warmup", dict(num_warmup_steps=2, num_training_steps=10, lr_end=1e-3, power=2.0)),
-             ("get_linear_schedule_with_warmup", dict(num_warmup_steps=2, num_training_steps=10)),
-             ("get_constant_schedule_with_warmup", dict(num_warmup_steps=2)), ("get_constant_schedule", {})]
-    for fn, kw in cases:
-        seqs = []
-        for mod in (ref, mine):
-            opt = torch.optim.SGD([torch.nn.Parameter(torch.zeros(1))], lr=0.5)
-            sch = getattr(mod, fn)(opt, **kw)
-            seq = []
-            for _ in range(12):
-                opt.step(); sch.step(); seq.append(sch.get_last_lr()[0])
-            seqs.append(seq)
-        assert seqs[0] == pytest.approx(seqs[1], rel=1e-12, abs=1e-15), fn
-    assert [e.value for e in mine.SchedulerType] == [e.value for e in ref.SchedulerType]
+    assert list(mine.NAMES) == list(ref["get_scheduler"])
+    for name, want in ref["get_scheduler"].items():
+        got = _lr_sequence(lambda o: mine.get_scheduler(name, optimizer=o, num_warmup_steps=3, num_training_steps=10))
+        assert got == pytest.approx(want, rel=1e-12, abs=1e-15), name
+    for fn, kw, want in ref["constructors"]:
+        assert _lr_sequence(lambda o: getattr(mine, fn)(o, **kw)) == pytest.approx(want, rel=1e-12, abs=1e-15), fn
+    assert [e.value for e in mine.SchedulerType] == ref["scheduler_types"]
     assert set(mine.TYPE_TO_SCHEDULER_FUNCTION) == set(mine.SchedulerType)
-    for k in [k for k in sys.modules if k.startswith("_ref_muse")]:
+    for k in [k for k in sys.modules if k == "muse" or k.startswith("muse.")]:
         del sys.modules[k]
 
 
+@needs_script
 @pytest.mark.parametrize("soft_targets", [False, True])
 def test_reference_training_script_trains_on_the_numeric_restatements(monkeypatch, tmp_path, soft_targets):
     """The same unmodified script with NUMERIC torch restatements of the kernels (tests/cpu_math_ops.py, precision-recipe
@@ -170,6 +159,7 @@ def test_reference_training_script_trains_on_the_numeric_restatements(monkeypatc
     assert ev and math.isfinite(ev[-1])
 
 
+@needs_script
 def test_reference_offline_ema_script_runs_unchanged(monkeypatch, tmp_path):
     """scripts/compute_offline_ema.py of the reference (load_config / from_pretrained over the checkpoint-N/unwrapped_model
     directories a training run leaves behind, EMAModel.step / copy_to, save_pretrained), unmodified, against the drop-in
@@ -217,6 +207,7 @@ def test_reference_offline_ema_script_runs_unchanged(monkeypatch, tmp_path):
         assert torch.equal(got[k], v), k
 
 
+@needs_script
 def test_reference_training_script_resumes_from_its_checkpoint(monkeypatch, tmp_path):
     """Checkpoint / resume of the unmodified script (train_maskgit_imagenet.py:329-355): a 4-step run that saved at step 2
     is resumed with ``experiment.resume_from_checkpoint=latest`` for two more steps -- model weights, AdamW moments and the
@@ -244,6 +235,7 @@ def test_reference_training_script_resumes_from_its_checkpoint(monkeypatch, tmp_
     assert int(next(iter(opt["state"].values()))["step"]) == 4  # AdamW's own step counter continued from the loaded state
 
 
+@needs_script
 def test_reference_benchmark_models_script_runs_unchanged(monkeypatch, tmp_path, capsys):
     """scripts/benchmark_models.py of the reference, unmodified (load_config / from_config, text-conditional generate2 in
     fp32, after ``model.half()`` and after enable_xformers_memory_efficient_attention(), timed with torch.utils.benchmark),
@@ -280,6 +272,7 @@ def test_reference_benchmark_models_script_runs_unchanged(monkeypatch, tmp_path,
     assert "Vanilla attention in FP32" in out and "Efficient attention in FP16" in out
 
 
+@needs_script
 def test_reference_training_script_with_gradient_accumulation(monkeypatch, tmp_path):
     """training.gradient_accumulation_steps = 2: the script's ``accelerator.accumulate(model)`` windows -- gradients of two
     micro-batches add up in the parameters' .grad (each per-layer Function hands its gradients to autograd's accumulation) and
